@@ -1,6 +1,6 @@
 """bench.py — headline benchmark of the B200 hot paths (contract: see the task statement / DESIGN.md §5).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 metric  : sampled edges/s of pyg_lib.sampler.neighbor_sample.
 N = 1   : BASELINE.json configs[1] — ogbn-products-shaped CSR (2,449,029 nodes / 123,718,280 edges, int64), fan-out
@@ -339,18 +339,53 @@ def load_traffic():
     return {k: sum(v) / len(v) for k, v in out.items()}
 
 
+DUMP_BYTES = 60 << 20   # stays under 64 MB (decimal) in all, .npy headers included
+
+
+def dump_outputs(out_dir, out):
+    """What a caller of (dist_)neighbor_sample receives, as float64 arrays (node and edge ids < 2^53 are exact).  A
+    result larger than DUMP_BYTES in all (a 65,536-seed batch) is written as a fixed sample: the same seeded, sorted
+    positions of row, col and edge_id (edge_positions.npy) and of node (node_positions.npy); the counts stay whole."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    row, col, node, eid, nph, eph = out
+    arrays = {'row': row, 'col': col, 'node': node, 'edge_id': eid}
+    n_e, n_n = row.size(0), node.size(0)
+    if 8 * (3 * n_e + n_n) > DUMP_BYTES:
+        keep = DUMP_BYTES / (8 * (4 * n_e + 2 * n_n))   # the position files count too
+
+        def positions(n):
+            g = torch.Generator().manual_seed(0)
+            return torch.randperm(n, generator=g)[:int(n * keep)].sort().values
+        pe, pn = positions(n_e), positions(n_n)
+        arrays = {'row': row.cpu()[pe], 'col': col.cpu()[pe], 'node': node.cpu()[pn], 'edge_id': eid.cpu()[pe],
+                  'edge_positions': pe, 'node_positions': pn}
+    arrays.update(num_sampled_nodes_per_hop=torch.tensor(nph), num_sampled_edges_per_hop=torch.tensor(eph))
+    for name, v in arrays.items():
+        np.save(osp.join(out_dir, name + '.npy'), v.cpu().numpy().astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=1000)
+    ap.add_argument('--steps', type=int, default=1000,
+                    help='timed steps of the headline path (N = 1: configs[1]; N > 1: configs[4] sharded), also of the N = 1 '
+                         'e2e and configs[4] legs; the other legs time at most 20-200 steps and report their own count')
     ap.add_argument('--warmup', type=int, default=20)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-matmul', action='store_true')
     ap.add_argument('--no-parity', action='store_true')
     ap.add_argument('--no-c5', action='store_true', help='N=1: skip the papers100M-shaped single-GPU leg')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the results of the headline path\'s last timed call to DIR/<name>.npy (float64; rank 0)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     a.warmup = max(a.warmup, 3)
+    if a.dump_outputs and a.impl != 'b200':
+        ap.error('--dump-outputs: only for this implementation')
     if a.impl == 'reference':
         return reference_arm(a)
 
@@ -399,11 +434,18 @@ def main():
         seeds_host = [perm[b * BATCH:(b + 1) * BATCH].clone().pin_memory() for b in my_batches]
         seeds_dev = [s.to(dev) for s in seeds_host]
         torch.manual_seed(12345)
+        last = [None]
 
         def step_dev(i):
-            return P.sampler.neighbor_sample(rowptr, col, seeds_dev[i], FANOUT)[0].numel()
+            o = P.sampler.neighbor_sample(rowptr, col, seeds_dev[i], FANOUT)
+            if a.dump_outputs:
+                last[0] = o
+            return o[0].numel()
         ms, edges, _, launches, clocks = T.run(step_dev, a.steps, a.warmup)
         value = edges / (ms * 1e-3)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, last[0])
+        last[0] = None
 
         # e2e: pinned seeds -> device and (row, col, edge_id, node_id) -> pinned host EVERY step, through the public API.  The
         # calls themselves cannot overlap (each consumes the CPU generator where the previous one left it, and returns its
@@ -620,18 +662,18 @@ def c5_leg(a, P, abi, T, torch, dev, world, rank, peaks, hbm_peak, peak_src, tra
     rowptr, col = lognormal_csr(C5_NODES, C5_EDGES, seed=1, device=dev)
     torch.cuda.synchronize()
     gen_s = time.time() - t0
-    steps = min(a.steps, 100)
+    steps = a.steps
     perm = torch.randperm(C5_NODES, generator=torch.Generator().manual_seed(2))
-    n_b = C5_NODES // C5_BATCH
-    seeds_host = [perm[(i % n_b) * C5_BATCH:((i % n_b) + 1) * C5_BATCH].clone().pin_memory() for i in range(steps + a.warmup + 8)]
+    n_seeds = min(steps + a.warmup + 8, C5_NODES // C5_BATCH)   # step i takes batch i % n_seeds: a batch is 512 KB here and on the device
+    seeds_host = [perm[i * C5_BATCH:(i + 1) * C5_BATCH].clone().pin_memory() for i in range(n_seeds)]
     seeds_dev = [s.to(dev) for s in seeds_host]
     del perm
 
     def single(i):
-        return P.sampler.neighbor_sample(rowptr, col, seeds_dev[i], FANOUT)
+        return P.sampler.neighbor_sample(rowptr, col, seeds_dev[i % n_seeds], FANOUT)
 
     def sharded(i):
-        return P.sampler.dist_neighbor_sample(rowptr, col, seeds_dev[i], FANOUT)
+        return P.sampler.dist_neighbor_sample(rowptr, col, seeds_dev[i % n_seeds], FANOUT)
     op = single if world == 1 else sharded
     out = {'graph_gen_s': gen_s, 'steps': steps}
     if world > 1:
@@ -655,7 +697,18 @@ def c5_leg(a, P, abi, T, torch, dev, world, rank, peaks, hbm_peak, peak_src, tra
                                   'error': 'parity gate failed: nothing was timed'}), flush=True)
             sys.exit(1)
     torch.manual_seed(999)
-    ms, edges, _, launches, clocks = T.run(lambda i: op(i)[0].numel(), steps, a.warmup)
+    last = [None]
+    keep = bool(a.dump_outputs) and world > 1 and rank == 0   # N > 1: the headline path; its result is the same on every rank
+
+    def step(i):
+        o = op(i)
+        if keep:
+            last[0] = o
+        return o[0].numel()
+    ms, edges, _, launches, clocks = T.run(step, steps, a.warmup)
+    if keep:
+        dump_outputs(a.dump_outputs, last[0])
+    last[0] = None
     out.update({'value': edges / (ms * 1e-3), 'unit': 'edges/s', 'ms_per_step': ms / steps, 'edges_per_step': edges / steps,
                 'clocks': clocks, 'gpu_launches': launches})
     # e2e: seeds from pinned host memory, the full result back to pinned host memory on every rank
@@ -663,7 +716,7 @@ def c5_leg(a, P, abi, T, torch, dev, world, rank, peaks, hbm_peak, peak_src, tra
     copier = HostCopier(torch, dev, [cap, cap, cap + C5_BATCH, cap], n_slots=2)
 
     def step_e2e(i):
-        s = seeds_host[i].to(dev, non_blocking=True)
+        s = seeds_host[i % n_seeds].to(dev, non_blocking=True)
         o = (P.sampler.neighbor_sample(rowptr, col, s, FANOUT) if world == 1 else P.sampler.dist_neighbor_sample(rowptr, col, s, FANOUT))[:4]
         copier.submit(o)
         return o[0].numel()
@@ -693,6 +746,7 @@ def c5_leg(a, P, abi, T, torch, dev, world, rank, peaks, hbm_peak, peak_src, tra
         ms1, ed1, _, _, _ = T.run(lambda i: single(i)[0].numel(), min(steps, 20), 3)
         out['single_gpu_edges_per_s'] = ed1 / (ms1 * 1e-3)
         out['single_gpu_ms_per_step'] = ms1 / min(steps, 20)
+        out['single_gpu_steps'] = min(steps, 20)
         out['speedup_vs_1gpu'] = out['value'] / out['single_gpu_edges_per_s']
         out['strong_scaling_efficiency'] = out['speedup_vs_1gpu'] / world
     del rowptr, col

@@ -1,5 +1,5 @@
 """Reference outputs for config-size parity gates.  TEST/BENCH INFRASTRUCTURE ONLY — run as a subprocess by
-tests/ (test_config_parity.py) and by bench.py's parity gate; never imported by the product.
+bench.py's parity gate (and by tests/test_refproc.py, which checks that plumbing); never imported by the product.
 
     python oracle/ref_parity.py SPEC.pt
 

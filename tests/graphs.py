@@ -418,6 +418,40 @@ def mag240m_shaped(scale: float, device='cpu', seed0: int = 10):
     return sizes, rowptr_d, col_d
 
 
+# Inputs of the config-size parity tests (tests/test_config_parity.py) and of the fixtures they compare with
+# (tests/golden/make_golden_config.py).  c4 and c5 draw their graphs from the CUDA generator of `device`.
+def config_c2_inputs():
+    """configs[1]: ogbn-products-shaped CSR (bench.py's graph) and three 1024-seed batches."""
+    n, e = 2_449_029, 123_718_280
+    rowptr, col = lognormal_csr(n, e, seed=1)
+    perm = torch.randperm(n, generator=torch.Generator().manual_seed(2))
+    return rowptr, col, [perm[b * 1024:(b + 1) * 1024].clone() for b in (0, 1, 2)]
+
+
+def config_c3_inputs():
+    """configs[2]: 64 relations, N = 2^20 ragged rows (one empty segment), 128 -> 128 bf16.  Returns (x, ptr, w)."""
+    N, K, M, B = 1 << 20, 128, 128, 64
+    g = torch.Generator().manual_seed(0)
+    x = torch.randn(N, K, generator=g).to(torch.bfloat16)
+    w = (torch.randn(B, K, M, generator=g) / K ** 0.5).to(torch.bfloat16)
+    return x, ragged_ptr(N, B, 100), w
+
+
+def config_c4_inputs(device):
+    """configs[3] at 0.1 scale: (sizes, rowptr_dict, col_dict, 1024 paper seeds)."""
+    sizes, rowptr_d, col_d = mag240m_shaped(0.1, device=device)
+    seed = torch.randperm(sizes['paper'], generator=torch.Generator().manual_seed(3))[:1024]
+    return sizes, rowptr_d, col_d, seed
+
+
+def config_c5_inputs(device):
+    """configs[4]'s graph and batch: papers100M-shaped CSR (111,059,956 nodes / 1,615,685,872 edges), 65,536 seeds."""
+    n, e = 111_059_956, 1_615_685_872
+    rowptr, col = lognormal_csr(n, e, seed=1, device=device)
+    seed = torch.randperm(n, generator=torch.Generator().manual_seed(2))[:65536]
+    return rowptr, col, seed
+
+
 # ------------------------------------------------------------------------------------- biased (edge_weight) sampling
 # graph / seeds as in HOMO_CASES; `weights`: how the float32 edge weights are drawn (build_weights)
 WEIGHTED_CASES: Dict[str, dict] = {

@@ -1,6 +1,8 @@
 """Run the reference (oracle/ref_parity.py, a subprocess: oracle/_ref/libpyg_ref.so and libpyg.so both register the
 pyg:: schemas) on inputs that may be too large to pickle: big tensors go through raw files under /dev/shm (or the
-temp dir) that the child maps with torch.from_file.  Used by tests/test_config_parity.py and bench.py's parity gate."""
+temp dir) that the child maps with torch.from_file.  Used by bench.py's parity gate; the comparison helpers below also
+serve tests/test_config_parity.py, which compares with stored outputs of the reference instead."""
+import hashlib
 import os
 import os.path as osp
 import shutil
@@ -75,6 +77,12 @@ def compare_homo(out, ref_call) -> dict:
 
 def rng_prefix():
     return torch.get_rng_state()[:24 + 624 * 8].clone()
+
+
+def sha256(t: torch.Tensor) -> bytes:
+    """SHA-256 of a tensor's elements in row-major order: how the config-size fixtures keep index tensors that are too
+    large to store (equal digests of same-shape, same-dtype tensors = bit-exact)."""
+    return hashlib.sha256(t.detach().cpu().contiguous().numpy().tobytes()).digest()
 
 
 def accumulation_bound(x: torch.Tensor, ptr: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
